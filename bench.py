@@ -9,8 +9,12 @@ work is fixed) -> parseOutput / 7-token de-interleave -> SNAC decode -> 8 wavefo
 ends with START_OF_SPEECH (128257, the first token a real checkpoint emits), so parseOutput crops the prompt as it
 does in a real run and the audio is BASELINE.md's 512 tokens -> 73 frames -> 6.229 s per utterance.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong] [--dump-outputs DIR]
     torchrun ... bench.py --gpus N ...          (one rank per GPU; utterances shard)
+
+Every block times K steps.  --dump-outputs DIR writes, after the timed steps, what each timed device path returned to its caller
+in its last step on rank 0 (DIR/<name>.npy: floating outputs as float32, integer ones as float64).  Inputs and weights are seeded,
+so two builds run with the same arguments can be compared output for output (DESIGN.md 5: which outputs repeat bit for bit).
 
 `value` : inputs already resident in HBM, waveforms left in HBM (b2a_tts_generate_dev).
 `e2e`   : same metric through the host-buffer C ABI call a user makes (b2a_tts_generate): pinned host ids
@@ -384,6 +388,24 @@ def whisper_encoder_flops() -> float:
     return float(conv + WHISPER_BASE["encoder_layers"] * layer)
 
 
+DUMP_BYTES_MAX = 64 << 20
+
+
+def write_outputs(directory, arrays: dict) -> None:
+    """DIR/<name>.npy for every array: float32 and narrower floats as float32, everything else (integers exactly) as float64."""
+    out = {}
+    for k, v in arrays.items():
+        v = np.asarray(v)
+        out[k] = v.astype(np.float32 if v.dtype.kind == "f" and v.itemsize <= 4 else np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BYTES_MAX:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES_MAX}-byte budget")
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    for k, a in out.items():
+        np.save(d / f"{k}.npy", a)
+
+
 def synth_clip(n: int, seed: int) -> np.ndarray:
     """SURVEY.md 8(d): x = 0.5 sin(2 pi 220 t) + 0.1 N(0, 1), clipped, 16 kHz."""
     rng = np.random.default_rng(seed)
@@ -420,7 +442,7 @@ class GpuTimer:
         return float(t.item()), self.m.launch_count() - n0, outs
 
 
-def whisper_block(m, torch, timer, rank, world, local, steps, warmup):
+def whisper_block(m, torch, timer, rank, world, local, steps, warmup, dump=None):
     """BASELINE config 3: Whisper-base, 16 x 30 s synthetic clips per GPU, greedy, 64 forced decode steps (EOT masked)."""
     wm = m.WhisperModel.random_init(WHISPER_BASE, device=local, max_batch=WH_BATCH)
     stream = torch.cuda.ExternalStream(wm.stream, device=torch.device("cuda", local))
@@ -430,6 +452,8 @@ def whisper_block(m, torch, timer, rank, world, local, steps, warmup):
     toks = torch.zeros((WH_BATCH, WH_STEPS), dtype=torch.int32).pin_memory()
     ntok = torch.zeros(WH_BATCH, dtype=torch.int32).pin_memory()
     ms_dev, launches, outs = timer(lambda: wm.generate_dev(pcm_dev, P, toks.numpy(), ntok.numpy()), stream, steps, warmup)
+    if dump is not None:
+        dump["whisper_tokens"], dump["whisper_token_counts"] = toks.numpy().copy(), ntok.numpy().copy()
     pcm_np = pcm_host.numpy()                       # a view of the pinned buffer: the C ABI copies host -> device from it
     ms_e2e, _, _ = timer(lambda: wm.generate(pcm_np, P), stream, steps, 1)
     assert int(ntok.min()) == WH_STEPS, "whisper benchmark produced too few tokens"
@@ -453,7 +477,7 @@ def whisper_block(m, torch, timer, rank, world, local, steps, warmup):
                          "(includes the log-mel kernel and the cross-K/V projections); log-mel algorithmic bytes %d per step" % alg_mel}}
 
 
-def snac_block(m, torch, timer, rank, world, local, codec, steps, warmup):
+def snac_block(m, torch, timer, rank, world, local, codec, steps, warmup, dump=None):
     """BASELINE config 2: SNAC-24kHz decode, batch 8 x 1024 latent steps -> 8 x 524 288 samples (21.85 s each)."""
     stream = torch.cuda.ExternalStream(codec.stream, device=torch.device("cuda", local))
     rng = np.random.default_rng(2 + rank)
@@ -461,6 +485,8 @@ def snac_block(m, torch, timer, rank, world, local, codec, steps, warmup):
     codes_dev = [c.cuda() for c in codes_host]
     wave_dev = torch.empty((SNAC_BATCH, 1, SNAC_T * 512), device="cuda")
     ms_dev, launches, _ = timer(lambda: codec.decode_dev(codes_dev, wave_dev, seed=1, stream=codec.stream), stream, steps, warmup)
+    if dump is not None:
+        dump["snac_waveforms"] = wave_dev.cpu().numpy()
     codes_np = [c.numpy() for c in codes_host]
     wave_np = torch.empty((SNAC_BATCH, 1, SNAC_T * 512), dtype=torch.float32).pin_memory().numpy()
     ms_e2e, _, outs = timer(lambda: codec.decode(codes_np, out=wave_np), stream, steps, 1)
@@ -485,7 +511,7 @@ def snac_block(m, torch, timer, rank, world, local, codec, steps, warmup):
 Q3_ROWS, Q3_FRAMES, Q3_CHUNK = 4, 1024, 64
 
 
-def qwen3_block(m, torch, timer, rank, world, local, steps, warmup):
+def qwen3_block(m, torch, timer, rank, world, local, steps, warmup, dump=None):
     """BASELINE config 5: Qwen3-TTS-0.6B geometry (talker 1024 x 28, code predictor 1024 x 5, 16 code groups; random-init bf16 -- an
     8-bit checkpoint is expanded to bf16 at load, DESIGN.md 3.9), batch 32 over 8 GPUs = 4 utterances per GPU, 1024 frames each
     (81.9 s of audio), the codes decoded by the speech-tokenizer decoder (the model's vocoder) in streaming chunks of 64 frames."""
@@ -503,7 +529,7 @@ def qwen3_block(m, torch, timer, rank, world, local, steps, warmup):
     pad = (0.05 * rng.standard_normal(H)).astype(np.float32)
     P = m.Qwen3GenerateParameters(max_tokens=Q3_FRAMES, temperature=0.9, top_k=50, top_p=1.0, repetition_penalty=1.05, seed=rank, mask_eos=True)
     stream = torch.cuda.ExternalStream(talker.stream, device=torch.device("cuda", local))
-    stages = {}
+    stages, last = {}, {}
 
     def step():
         t0 = time.perf_counter()
@@ -511,14 +537,15 @@ def qwen3_block(m, torch, timer, rank, world, local, steps, warmup):
         t1 = time.perf_counter()
         c = np.ascontiguousarray(np.stack(codes).transpose(0, 2, 1))                    # [B, 16, frames]
         dec.reset_streaming_state()
-        n = 0
-        for f0 in range(0, Q3_FRAMES, Q3_CHUNK):
-            n += dec.streaming_step(c[:, :, f0:f0 + Q3_CHUNK]).shape[-1]
+        audio = [dec.streaming_step(c[:, :, f0:f0 + Q3_CHUNK]) for f0 in range(0, Q3_FRAMES, Q3_CHUNK)]
         stages["talker"], stages["decoder"] = t1 - t0, time.perf_counter() - t1
-        assert n == Q3_FRAMES * 1920 and all(len(x) == Q3_FRAMES for x in codes)
+        assert sum(a.shape[-1] for a in audio) == Q3_FRAMES * 1920 and all(len(x) == Q3_FRAMES for x in codes)
+        last["codes"], last["audio"] = c, audio
         return info
 
     ms, launches, infos = timer(step, stream, steps, warmup)           # every call ends synchronised (codes / audio copied to the host)
+    if dump is not None:
+        dump["qwen3_codes"], dump["qwen3_audio"] = last["codes"], np.concatenate(last["audio"], axis=-1)
     audio = Q3_ROWS * Q3_FRAMES * 1920 / 24000.0 * world
     frame_ms = float(np.median([i.generate_time for i in infos])) / Q3_FRAMES * 1e3
     return {"metric": "qwen3tts_0.6b_rtfx_batch4_per_gpu", "unit": UNIT, "value": audio * steps / (ms * 1e-3), "ms_per_step": ms / steps,
@@ -547,7 +574,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the whisper / snac blocks")
     ap.add_argument("--tiny", action="store_true", help="small model (plumbing check only; NOT a bench number)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what each timed device path returned in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
 
@@ -591,12 +621,15 @@ def main():
     wave_dev = torch.zeros((rows, wave_len), dtype=torch.float32, device="cuda")
     gathered = torch.zeros((world, rows, wave_len), dtype=torch.float32, device="cuda") if world > 1 else None
     stream = torch.cuda.ExternalStream(tts.stream, device=torch.device("cuda", local))
+    dump = {} if args.dump_outputs and rank == 0 else None
+    last = {}
 
     def step_dev():
         wl, info = tts.generate_dev(ids_dev, params, wave_dev, wave_len)
         if dist is not None:      # the ONE collective of the path: re-join decoded waveforms
             with torch.cuda.stream(stream):
                 dist.all_gather_into_tensor(gathered, wave_dev)
+        last["wave_lengths"] = wl
         return info
 
     def step_e2e():
@@ -607,6 +640,8 @@ def main():
         sampler.start()
     ms_dev, launches, infos = timer(step_dev, stream, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if dump is not None:
+        dump["orpheus_waveforms"], dump["orpheus_wave_lengths"] = wave_dev.cpu().numpy(), last["wave_lengths"]
     ms_e2e, _, _ = timer(step_e2e, stream, args.steps, max(1, min(args.warmup, 1)))
     assert int(wlen_host[0]) == wave_len and bool(torch.isfinite(wave_host).all()), "benchmark produced no / bad audio"
 
@@ -624,10 +659,10 @@ def main():
     if not args.no_secondary and not args.tiny:
         del tts
         torch.cuda.empty_cache()
-        secondary["whisper"] = whisper_block(m, torch, timer, rank, world, local, max(3, min(args.steps, 10)), 3)
-        secondary["snac"] = snac_block(m, torch, timer, rank, world, local, codec, max(3, min(args.steps, 10)), 3)
+        secondary["whisper"] = whisper_block(m, torch, timer, rank, world, local, args.steps, 3, dump)
+        secondary["snac"] = snac_block(m, torch, timer, rank, world, local, codec, args.steps, 3, dump)
         try:
-            secondary["qwen3"] = qwen3_block(m, torch, timer, rank, world, local, 2, 1)
+            secondary["qwen3"] = qwen3_block(m, torch, timer, rank, world, local, args.steps, 1, dump)
         except Exception as e:      # row N1 is the newest path: the headline line must still print
             secondary["qwen3"] = {"unavailable": repr(e)[:300]}
 
@@ -635,6 +670,8 @@ def main():
         if dist is not None:
             dist.destroy_process_group()
         return
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     value = world * audio_s * args.steps / (ms_dev * 1e-3)
     e2e = world * audio_s * args.steps / (ms_e2e * 1e-3)
     traffic = MEASURED_STEP_DRAM_BYTES["bytes"] if (rows == MEASURED_STEP_DRAM_BYTES["batch"] and not args.tiny) else None

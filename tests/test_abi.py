@@ -128,3 +128,25 @@ def test_bench_workload_accounting():
     assert abs((bench.weight_bytes(cfg) + bench.kv_bytes(cfg, 8, 320, 2)) / 1e9 - 6.895) < 1e-3
     assert bench.bench_config(cfg, 4, "weak")["global_batch"] == 32 and bench.bench_config(cfg, 4, "strong")["global_batch"] == 8
     assert bench.bench_config(cfg, 8, "strong")["rows_per_gpu"] == 1
+
+
+def test_bench_output_dump(tmp_path, monkeypatch):
+    """--dump-outputs: one float32 / float64 .npy per output (integers exactly as float64), a bounded total, and a step count that
+    is really used (no zero-step run)."""
+    import sys
+    sys.path.insert(0, str(ROOT))
+    import bench
+    wave = np.random.default_rng(0).standard_normal((2, 5)).astype(np.float32)
+    lens = np.array([5, 2**40 + 1], dtype=np.int64)
+    bench.write_outputs(tmp_path / "d", {"wave": wave, "lens": lens, "half": wave.astype(np.float16)})
+    got = {p.stem: np.load(p) for p in (tmp_path / "d").glob("*.npy")}
+    assert set(got) == {"wave", "lens", "half"}
+    assert got["wave"].dtype == np.float32 and np.array_equal(got["wave"], wave)
+    assert got["lens"].dtype == np.float64 and got["lens"].astype(np.int64).tolist() == lens.tolist()
+    assert got["half"].dtype == np.float32
+    with pytest.raises(ValueError):
+        bench.write_outputs(tmp_path / "big", {"x": np.zeros(bench.DUMP_BYTES_MAX // 4 + 1, np.float32)})
+    assert not (tmp_path / "big").exists()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.main()
